@@ -5,6 +5,7 @@
     python bench.py --workload md17_egnn|oc20_mace|gfm_pnaeq|lj_egnn   # the other BASELINE.json configs (SURVEY 8d C3/C4/C5/C1)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1     # CPU arm (oracle on the host cores)
+    python bench.py --steps 20 --warmup 5 --dump-outputs DIR           # + what the last timed step computed, as DIR/<name>.npy
 
 One "step" = neighbour build (radius graph, periodic for C1/C4, + CSR plans) -> forward -> loss -> backward -> flat gradient
 all-reduce -> fused AdamW on one batch.  Weak scaling: every rank owns ``--graphs`` graphs per step; ``value`` = atoms processed
@@ -63,6 +64,9 @@ def parse():
     ap.add_argument("--ref-graphs", type=int, default=None, help="graphs per step of the CPU arm / cpu_baseline sample")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-kernel-shares", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, per-task losses, head predictions, flat "
+                         "gradient, parameters after the update) as DIR/<name>.npy in float32 (rank 0)")
     ap.add_argument("--precision", default=None, choices=["bf16", "fp32"],
                     help="bf16 = tensor-core (tcgen05, TF32-in/fp32-acc) Linears; fp32 = exact SIMT kernels; default: the config's")
     a = ap.parse_args()
@@ -368,15 +372,17 @@ def run_engine(args):
         m = model.module
         if mlip:
             d.pos.requires_grad_(True)
-            loss, _ = m.energy_force_loss(model(d), d)
+            pred = model(d)
+            loss, tasks = m.energy_force_loss(pred, d)
         else:
-            loss, _ = m.loss(model(d), d.y, hi)
+            pred = model(d)
+            loss, tasks = m.loss(pred, d.y, hi)
         flat = opt.backward(loss)
         if with_opt:
             if ws > 1 and collective:
                 dist.all_reduce(flat)
             opt.step(1.0 / ws)
-        return loss.detach()
+        return loss.detach(), [t.detach() for t in tasks], [p.detach() for p in pred]
 
     # eager warm-up (also measures the sizes per batch and the number of libhgb launches per step)
     sizes = []
@@ -392,7 +398,7 @@ def run_engine(args):
     launches_per_step = _lib.launch_count() - c0
 
     use_graph = not args.no_graph
-    graphs, losses, g_opt = [], [], None
+    graphs, outs, g_opt = [], [], None
     if use_graph:
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
@@ -405,9 +411,9 @@ def run_engine(args):
         for d, hi, sz in zip(devb, hidx, sizes):
             g = torch.cuda.CUDAGraph()
             with ops.capture_graph(g):
-                l = step(d, hi, known=sz, with_opt=one_graph)
+                out = step(d, hi, known=sz, with_opt=one_graph)
             graphs.append(g)
-            losses.append(l)
+            outs.append(out)
         if not one_graph:
             g_opt = torch.cuda.CUDAGraph()
             with ops.capture_graph(g_opt):
@@ -419,7 +425,7 @@ def run_engine(args):
     copy_stream = torch.cuda.Stream()
     ready = [torch.cuda.Event() for _ in range(args.nbatches)]      # inputs of batch b are on the device
     released = [torch.cuda.Event() for _ in range(args.nbatches)]   # the step that used batch b has been enqueued and finished
-    state = {"prefetched": -1}
+    state = {"prefetched": -1, "last": None}
 
     def issue_copy(i):
         b = i % args.nbatches
@@ -445,12 +451,13 @@ def run_engine(args):
             if g_opt is not None:
                 dist.all_reduce(opt.flat_g)
                 g_opt.replay()
-            l = losses[b]
+            out = outs[b]
         else:
-            l = step(d, hidx[b], known=sizes[b])
+            out = step(d, hidx[b], known=sizes[b])
+        state["last"] = out                     # (loss, per-task losses, predictions) of this step
         if e2e:
             released[b].record()
-            loss_host.copy_(l.reshape(1), non_blocking=True)
+            loss_host.copy_(out[0].reshape(1), non_blocking=True)
             if args.nbatches > 1:
                 issue_copy(i + 1)
 
@@ -517,6 +524,8 @@ def run_engine(args):
     torch.cuda.synchronize()
     ops.check_guard(dev)                                     # every captured neighbour build produced the promised edge count
     clocks = sampler.stop() if sampler else None
+    if rank == 0 and args.dump_outputs:                      # before the profiled step below moves the parameters on
+        dump_outputs(args.dump_outputs, state["last"], opt)
     value = atoms_all / K / (ms_dev * 1e-3)
     e2e = atoms_all / K / (ms_e2e * 1e-3)
 
@@ -567,14 +576,37 @@ def run_engine(args):
     _shutdown(ws, dev, [graphs, g_opt])
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, out, opt):
+    """Write what one training step returned to its caller (loss, per-task losses, every head's prediction) and what it left in
+    the optimizer (flat gradient, parameters after the update) as float32 ``path/<name>.npy``.  An array larger than its share
+    of DUMP_BYTES is replaced by a fixed, seeded sample of its elements, flattened, in index order."""
+    import numpy as np
+    loss, tasks, pred = out
+    arrays = {"loss": loss.reshape(1), "tasks_loss": torch.stack(tasks), "grads": opt.flat_g, "params": opt.flat_p}
+    arrays.update(("pred_%d" % i, p) for i, p in enumerate(pred))
+    cap = DUMP_BYTES // 4 // len(arrays)
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def _shutdown(ws, dev, keep_alive):
-    """Leave without tearing NCCL down: destroying a process group whose collectives live inside captured CUDA graphs can block
-    forever at interpreter exit (observed: the 2-GPU run printed its line and then hung in teardown).  Every rank drains its GPU,
-    meets the others once, flushes and exits the process directly."""
+    """One process: drain the GPU and return, so the interpreter shuts down normally and its exit handlers run.
+    Several ranks: leave without tearing NCCL down: destroying a process group whose collectives live inside captured CUDA graphs
+    can block forever at interpreter exit (observed: the 2-GPU run printed its line and then hung in teardown).  Every rank drains
+    its GPU, meets the others once, flushes and exits the process directly."""
     torch.cuda.synchronize()
-    if ws > 1:
-        dist.barrier()
-        torch.cuda.synchronize()
+    if ws == 1:
+        return
+    dist.barrier()
+    torch.cuda.synchronize()
     sys.stdout.flush()
     sys.stderr.flush()
     os._exit(0)

@@ -422,7 +422,7 @@ def main():
     from oracle.gps import PyGBatchNorm
     sys.modules["hydragnn.models.Base"].BatchNorm = PyGBatchNorm
     gen2 = torch.Generator().manual_seed(4321)
-    hmodels = {}
+    hmodels, hmodels64 = {}, {}
     heads_pernode = {"node": [{"type": "branch-0", "architecture": {"num_headlayers": 2, "dim_headlayers": [7, 5], "type": "mlp_per_node"}}]}
     heads_conv = {"node": [{"type": "branch-0", "architecture": {"num_headlayers": 2, "dim_headlayers": [10, 6], "type": "conv"}}]}
     for name in ("egnn_mlp_per_node", "egnn_conv_head", "painn_conv_head"):
@@ -446,7 +446,17 @@ def main():
         grads = torch.autograd.grad(loss, list(m.parameters()), allow_unused=True)
         hmodels[name] = {"state": state, "inputs": t2d(b), "pred": [p.detach() for p in pred], "loss": loss.detach(),
                          "grads": {n: (g.detach() if g is not None else None) for (n, _), g in zip(m.named_parameters(), grads)}}
+        # the same weights and inputs in fp64: a conv head's batch-statistics BatchNorm over a few nodes amplifies fp32 rounding
+        # to ~1e-5 relative, by an amount that depends on the host's BLAS kernels and thread count
+        m.double()
+        b64 = b.clone().to(dtype=torch.float64)
+        pred = m(b64)
+        loss, _ = m.loss(pred, b64.y, [torch.arange(b64.y.shape[0])])
+        grads = torch.autograd.grad(loss, list(m.parameters()), allow_unused=True)
+        hmodels64[name] = {"pred": [p.detach() for p in pred], "loss": loss.detach(),
+                           "grads": {n: (g.detach() if g is not None else None) for (n, _), g in zip(m.named_parameters(), grads)}}
     torch.save(hmodels, HERE + "/models_heads.pt")
+    torch.save(hmodels64, HERE + "/models_heads_fp64.pt")
 
     # ---- MACE through the reference's own MACEStack / blocks / symmetric_contraction / cg / irreps_tools (e3nn restated) ----
     mace = install_mace_stubs()

@@ -57,7 +57,7 @@ def test_missing_library_fails_loudly(monkeypatch):
 def test_create_model_reproduces_reference_initialisation(golden_dir):
     g = torch.load(golden_dir + "/models.pt")
     for name, kw in MODEL_KW.items():
-        sd = hb.create_model(**kw).state_dict()
+        sd = hb.create_model(use_gpu=False, **kw).state_dict()
         assert list(sd.keys()) == list(g[name]["state"].keys()), name
         for k, v in sd.items():
             assert torch.equal(v, g[name]["state"][k]), (name, k)
@@ -66,7 +66,7 @@ def test_create_model_reproduces_reference_initialisation(golden_dir):
 def test_pnaeq_initialisation_matches_reference(golden_dir):
     g = torch.load(golden_dir + "/models_pnaeq.pt")
     for name, c in g.items():
-        sd = hb.create_model(**dict(PNAEQ_KW, graph_pooling=name.split("_")[-1], pna_deg=c["deg"])).state_dict()
+        sd = hb.create_model(use_gpu=False, **dict(PNAEQ_KW, graph_pooling=name.split("_")[-1], pna_deg=c["deg"])).state_dict()
         assert list(sd.keys()) == list(c["state"].keys())
         for k, v in sd.items():
             assert torch.equal(v, c["state"][k]), (name, k)
@@ -77,7 +77,7 @@ def test_pnaeq_initialisation_matches_reference(golden_dir):
 def test_gps_initialisation_matches_reference(golden_dir):
     g = torch.load(golden_dir + "/models_gps.pt")
     for name, c in g.items():
-        sd = hb.create_model(**GPS_KW[name]).state_dict()
+        sd = hb.create_model(use_gpu=False, **GPS_KW[name]).state_dict()
         assert list(sd.keys()) == list(c["state"].keys())
         for k, v in sd.items():
             assert torch.equal(v, c["state"][k]), (name, k)
